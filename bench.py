@@ -7,6 +7,7 @@ reprojection loss, the selected train op (MAD module / FULL) with its momentum u
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config C] [--batch B]   # this framework (CUDA, libmadstereo)
   python bench.py --impl reference ...                                          # the reference path on host cores
+  python bench.py ... --dump-outputs DIR     # also write what the last timed step computed to DIR/*.npy (dump_outputs)
 
   --config 3 (default, the headline of BASELINE.json): MADNet + MAD (SEQUENTIAL sampler), 1280x384, 1 frame / GPU
            1: MADNet forward only, 640x384         2: MADNet FULL back-prop, 1280x384
@@ -241,6 +242,30 @@ def run_reference(args, cfg):
 # ---------------------------------------------------------------------------------------------------
 # this framework
 # ---------------------------------------------------------------------------------------------------
+DUMP_MAX_ELEMS = 4 << 20         # per array: at most 16 MB of float32, so a dump stays far below 64 MB
+
+
+def dump_outputs(dirname, step, disp, weights):
+    """What the last timed step handed its caller, one .npy per array, so that two builds can be compared output for
+    output: loss.npy and train_loss.npy (float64 [1]), blocks.npy (the MAD modules it trained, float64), disparity.npy
+    (the full-resolution disparity [B,H,W,1], float32) and weights.npy (the adapted weights, the engine's flat float32
+    parameter arena).  An array above DUMP_MAX_ELEMS is replaced by a fixed seeded sample of that many elements
+    (flattened, ascending index), the same for every run with the same arguments."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+
+    def put(name, a):
+        if a.size > DUMP_MAX_ELEMS:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(dirname, name + '.npy'), a)
+
+    put('loss', np.array([step['loss']], dtype=np.float64))
+    put('train_loss', np.array([step['train_loss']], dtype=np.float64))
+    put('blocks', np.array(step['blocks'], dtype=np.float64))
+    put('disparity', disp.detach().float().cpu().numpy())
+    put('weights', weights.detach().float().cpu().numpy())
+
+
 def parity_check(cfg, net, ad, eng, frame):
     """Engine forward on the first frame vs the CPU oracle with the SAME weights; returns the worst relative L-inf over
     the disparity outputs.  Checker only (outside every timed region)."""
@@ -330,15 +355,13 @@ def run_ours(args, cfg):
 
     disp_host = torch.empty(B, H, W, 1, dtype=torch.float32).pin_memory()
     full_disp = net.get_disparities()[-1]
+    last = {}
 
     def timed(src, steps, warmup, pipelined=False, fetch_disp=False):
         # pipelined: the host->device copy of frame i+1 is issued (side stream) while frame i computes; every frame's
         # copy is still inside the timed region
         def one(i):
-            if pipelined:
-                ad.step(*src[i % n_sets], prefetch=src[(i + 1) % n_sets])
-            else:
-                ad.step(*src[i % n_sets])
+            last['step'] = ad.step(*src[i % n_sets], prefetch=src[(i + 1) % n_sets] if pipelined else None)
             if fetch_disp:
                 disp_host.copy_(full_disp.tensor(), non_blocking=True)
         for i in range(warmup):
@@ -363,6 +386,8 @@ def run_ours(args, cfg):
     if clk:
         clk.start()
     ms_dev, launches = timed(dev_pairs, args.steps, args.warmup)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last['step'], full_disp.tensor(), eng.weights)
     ms_e2e_serial, _ = timed(host_pairs, args.steps, 3)
     ms_e2e, _ = timed(host_pairs, args.steps, 3, pipelined=True)
     ms_e2e_disp, _ = timed(host_pairs, args.steps, 3, pipelined=True, fetch_disp=True)
@@ -507,7 +532,11 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-parity-check', action='store_true')
     ap.add_argument('--no-corr-shapes', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed as DIR/<name>.npy (rank 0; see dump_outputs)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     cfg = CONFIGS[args.config]
     if args.impl == 'reference':
         return run_reference(args, cfg)
