@@ -61,19 +61,9 @@ int ms_conv2d_fwd(const float* x, int n, int h, int w, int cin, int x_cs, const 
 int ms_conv2d_dgrad(const float* dy, int n, int oh, int ow, int cout, int dy_cs, const float* weights,
                     float* dx, int h, int w, int cin, int dx_cs, int kh, int kw, int stride, int dilation,
                     float* scratch, void* stream);
-/* tcgen05 (5th-gen tensor core, 3xTF32 split => fp32-grade accuracy) variants of the two ops above for
- * stride-1 convolutions; the engine uses them automatically for eligible layers (MS_CONV_TC=0 disables).
- * scratch: ms_conv2d_tc_scratch() floats.  Returns -3 if the shape is not eligible. */
-int ms_conv2d_fwd_tc(const float* x, int n, int h, int w, int cin, int x_cs, const float* weights /*HWIO*/,
-                     const float* bias, float* y, int cout, int y_cs, int kh, int kw, int dilation, float alpha,
-                     float* scratch, size_t scratch_floats, void* stream);
-int ms_conv2d_dgrad_tc(const float* dy, int n, int h, int w, int cout, int dy_cs, const float* weights /*HWIO*/,
-                       float* dx, int cin, int dx_cs, int kh, int kw, int dilation, float* scratch,
-                       size_t scratch_floats, void* stream);
-size_t ms_conv2d_tc_scratch(int kh, int kw, int cin, int cout);
-/* Split-16-bit tcgen05 path (csrc/conv_bf.cu; the engine's default for every eligible layer, MS_CONV_IMPL=tf32 selects
- * the 3xTF32 kernels above): operands as two 16-bit planes (x ~= hi + lo), three kind::f16 MMAs per K step at the
- * bf16/fp16 tensor rate.  Forward operands are fp16 planes of x * act_scale and of w (22 mantissa bits, ~2^-22 relative
+/* Split-16-bit tcgen05 path (csrc/conv_bf.cu; the engine's implementation of every eligible layer): operands as two
+ * 16-bit planes (x ~= hi + lo), three kind::f16 MMAs per K step at the bf16/fp16 tensor rate.  Forward operands are
+ * fp16 planes of x * act_scale and of w (22 mantissa bits, ~2^-22 relative
  * product error; the power-of-two scale is undone exactly in the epilogue); gradient operands are bf16 planes (16 bits, fp32 exponent
  * range).  GEMM transposed so that M = output channels and N = up to 256 pixels, halo patches by TMA (64-channel K
  * blocks), pre-tiled weights by 1-D bulk copies, stride 1 or 2 (TMA element strides), any dilation, split-K reduced by
@@ -118,7 +108,8 @@ int ms_conv2d_wgrad_bf_planes(const void* xhi, const void* xlo, int x_pcs, int n
                               const void* dhi, const void* dlo, int d_pcs, int oh, int ow, int cout, float* dw, float* db,
                               int kh, int kw, int stride, int dilation, float* workspace, size_t workspace_floats, void* stream);
 size_t ms_conv2d_wgrad_bf_workspace(int kh, int kw, int cin, int cout);
-/* tcgen05 weight gradient of a stride-1 conv (same outputs as ms_conv2d_wgrad); workspace from ..._workspace(). */
+/* 3xTF32 tcgen05 weight gradient of a stride-1 conv (same outputs as ms_conv2d_wgrad); the engine uses it for the layers
+ * whose output gradient has no bf16 planes.  workspace from ..._workspace().  -3 = not eligible. */
 int ms_conv2d_wgrad_tc(const float* x, int n, int h, int w, int cin, int x_cs, const float* dy, int cout, int dy_cs,
                        float* dw /*HWIO*/, float* db, int kh, int kw, int dilation, float* workspace,
                        size_t workspace_floats, void* stream);
@@ -259,9 +250,6 @@ float ms_engine_profile_event_overhead_ms(void* e);
 int ms_engine_profile_read(void* e, double* ms7, double* macs7, double* bytes7, long long* calls7);
 /* Kernels launched by this library in this process so far. */
 long long ms_launch_count(void);
-/* Diagnostic (no reference counterpart): per-role clock64 counters of the tcgen05 conv kernel, filled only when the
- * environment selects its profiling build (MS_TC_DEBUG=8, scripts/tc_prof.py). out32: 32 counters; reset != 0 clears. */
-int ms_debug_tc_prof(unsigned long long* out32, int reset);
 /* Diagnosis: cycles per tcgen05.mma.kind::f16 (M = 128, K = 16, bf16) issued back to back by one thread per CTA on zeroed
  * shared memory, for K-major / MN-major operand layouts, MMA N, number of accumulators visited round-robin, and the
  * issue scheme (uni = 0: loop on lane 0 only; 1: warp-uniform loop, elected lane issues).  out_dev:

@@ -26,7 +26,7 @@ static void copy_str(char* dst, int cap, const std::string& s) {
 
 extern "C" {
 
-int ms_version(void) { return 100; }
+int ms_version(void) { return 101; }
 const char* ms_last_error(void) { return ms::last_error_cstr(); }
 
 int ms_corr_fwd(const float* left, int left_cs, const float* right, int right_cs, const float* u, int u_cs,
@@ -98,36 +98,6 @@ int ms_conv2d_dgrad(const float* dy, int n, int oh, int ow, int cout, int dy_cs,
     return conv_gemm(p, S(stream));
 }
 
-int ms_conv2d_fwd_tc(const float* x, int n, int h, int w, int cin, int x_cs, const float* weights, const float* bias,
-                     float* y, int cout, int y_cs, int kh, int kw, int dilation, float alpha, float* scratch,
-                     size_t scratch_floats, void* stream) {
-    int oh, ow, pt, pl;
-    same_pad_c(h, kh, 1, dilation, oh, pt);
-    same_pad_c(w, kw, 1, dilation, ow, pl);
-    ConvGemm p{};
-    p.x = view(const_cast<float*>(x), n, h, w, cin, x_cs);
-    p.y = view(y, n, oh, ow, cout, y_cs);
-    p.wmat = weights; p.bias = bias; p.kh = kh; p.kw = kw;
-    p.mul = 1; p.off_y = -pt; p.off_x = -pl; p.step = dilation; p.div = 1;
-    p.alpha = alpha; p.mask = nullptr; p.mask_alpha = 1.f; p.res = nullptr; p.accumulate = 0;
-    if (!conv_tc_supported(p)) { set_error("ms_conv2d_fwd_tc: shape not supported by the tcgen05 path"); return -3; }
-    return conv_tc_oneshot(p, 0, scratch, scratch_floats, S(stream));
-}
-int ms_conv2d_dgrad_tc(const float* dy, int n, int h, int w, int cout, int dy_cs, const float* weights, float* dx,
-                       int cin, int dx_cs, int kh, int kw, int dilation, float* scratch, size_t scratch_floats,
-                       void* stream) {
-    int oh, ow, pt, pl;
-    same_pad_c(h, kh, 1, dilation, oh, pt);
-    same_pad_c(w, kw, 1, dilation, ow, pl);
-    ConvGemm p{};
-    p.x = view(const_cast<float*>(dy), n, h, w, cout, dy_cs);
-    p.y = view(dx, n, h, w, cin, dx_cs);
-    p.wmat = weights; p.bias = nullptr; p.kh = kh; p.kw = kw;
-    p.mul = 1; p.off_y = pt; p.off_x = pl; p.step = -dilation; p.div = 1;
-    p.alpha = 1.f; p.mask = nullptr; p.mask_alpha = 1.f; p.res = nullptr; p.accumulate = 0;
-    if (!conv_tc_supported(p)) { set_error("ms_conv2d_dgrad_tc: shape not supported by the tcgen05 path"); return -3; }
-    return conv_tc_oneshot(p, 1, scratch, scratch_floats, S(stream));
-}
 int ms_conv2d_fwd_bf(const float* x, int n, int h, int w, int cin, int x_cs, const float* weights, const float* bias,
                      float* y, int cout, int y_cs, int kh, int kw, int stride, int dilation, float alpha, float act_scale,
                      void* scratch, size_t scratch_bytes, void* stream) {
@@ -343,10 +313,6 @@ int ms_conv2d_wgrad_bf_planes(const void* xhi, const void* xlo, int x_pcs, int n
     return wgrad_bf(q, xp, dp, S(stream));
 }
 size_t ms_conv2d_wgrad_bf_workspace(int kh, int kw, int cin, int cout) { return wgrad_bf_workspace_floats(kh, kw, cin, cout); }
-size_t ms_conv2d_tc_scratch(int kh, int kw, int cin, int cout) {
-    size_t a = conv_tc_scratch_floats(kh * kw, cout, cin), b = conv_tc_scratch_floats(kh * kw, cin, cout);
-    return a > b ? a : b;
-}
 
 size_t ms_conv2d_wgrad_workspace(int kh, int kw, int cin, int cout, size_t out_pixels) {
     return conv_wgrad_workspace_floats(kh * kw, cin, cout, out_pixels);
@@ -502,9 +468,6 @@ int ms_engine_bind(void* h, float* weights, float* grads, float* momentum, float
     if (e->layout(workspace) > need) { set_error("ms_engine_bind: layout exceeds the size reported by ms_engine_sizes"); return -2; }
     MS_CHECK_CUDA(cudaMemsetAsync(workspace, 0, need * sizeof(float), S(stream)));
     MS_CHECK_CUDA(cudaMemsetAsync(grads, 0, e->n_params * sizeof(float), S(stream)));
-    if (!e->prep_jobs.empty())
-        MS_CHECK_CUDA(cudaMemcpyAsync(e->prep_jobs_dev, e->prep_jobs.data(), e->prep_jobs.size() * sizeof(TcPrepJob),
-                                      cudaMemcpyHostToDevice, S(stream)));
     if (!e->bf_jobs.empty())
         MS_CHECK_CUDA(cudaMemcpyAsync(e->bf_jobs_dev, e->bf_jobs.data(), e->bf_jobs.size() * sizeof(BfPrepJob),
                                       cudaMemcpyHostToDevice, S(stream)));
@@ -606,7 +569,6 @@ int ms_engine_profile_layers(void* h, double* ms3n, long long* calls3n) {
 }
 float ms_engine_profile_event_overhead_ms(void* h) { return static_cast<Engine*>(h)->prof_event_overhead_ms; }
 long long ms_launch_count(void) { return ms::launch_count(); }
-int ms_debug_tc_prof(unsigned long long* out32, int reset) { return ms::conv_tc_read_prof(out32, reset); }
 int ms_debug_bf_prof(unsigned long long* out, int max_ctas) { return ms::conv_bf_read_prof(out, max_ctas); }
 int ms_engine_num_tensors(void* h) { return (int)static_cast<Engine*>(h)->tensors.size(); }
 int ms_engine_tensor_name(void* h, int i, char* name, int cap) {

@@ -96,6 +96,7 @@ struct ConvGemm {
     int ksplit;           // set by conv_gemm()
 };
 int conv_gemm(const ConvGemm& p, cudaStream_t st);
+size_t conv_gemm_part_floats();      // size of the split-K scratch the engine passes as ConvGemm::part
 
 struct ConvWgrad {
     TView x;              // forward-conv input   [n, xh, xw, ci]
@@ -144,6 +145,7 @@ struct CorrFwd {
                                      // tensor-core kernel for wide windows (corr_mma.cu); 0: CUDA-core kernels only
 };
 int corr_fwd(const CorrFwd& p, cudaStream_t st);
+int corr_init();
 int mma_probe(int a_mn, int b_mn, int n, int n_acc, int rot, int iters, int uni, int ctas, long long* out_dev, cudaStream_t st);   // wgrad_bf.cu (diagnosis)
 bool corr_mma_supported(const CorrFwd& p);          // corr_mma.cu: wide window (>= 17 displacements), no warp, stride 1
 int corr_mma(const CorrFwd& p, cudaStream_t st);
@@ -207,26 +209,12 @@ int momentum_update(float* w, const float* g, float* m, size_t n, float lr, floa
 }  // namespace ms
 
 namespace ms {
-// tcgen05 path (conv_tc.cu)
-struct TcPrepJob {
-    const float* src; float* bh; float* bl;
-    int taps, N, K, BN, Kpad, transposed_src;
-};
-bool conv_tc_supported(const ConvGemm& g);
-void conv_tc_weight_dims(int N, int K, int& BN, int& Kpad);
-size_t conv_tc_scratch_floats(int taps, int N, int K);
-int conv_tc_init();
-int tc_prep_weights(const TcPrepJob* jobs_dev, int njobs, size_t max_total, cudaStream_t st);
-int conv_tc(const ConvGemm& g, const float* bw, cudaStream_t st, float* part);
-size_t conv_tc_part_floats();
-bool conv_tc_profitable(const ConvGemm& g);
-int conv_tc_oneshot(const ConvGemm& g, int wmat_is_nk, float* scratch, size_t scratch_floats, cudaStream_t st);
-int corr_init();
+// 3xTF32 tcgen05 weight gradient of stride-1 convolutions (wgrad_tc.cu): the engine's weight gradient for the shapes the
+// split-bf16 kernel does not take (DispNet's conv_redir, whose output gradient is a channel slice without bf16 planes)
 bool wgrad_tc_supported(const ConvWgrad& q);
 size_t wgrad_tc_workspace_floats(int taps, int ci, int co, int n, int h, int w);
 int wgrad_tc_init();
 int wgrad_tc(const ConvWgrad& q, cudaStream_t st);
-int conv_tc_read_prof(unsigned long long* out32, int reset);
 }  // namespace ms
 
 namespace ms {

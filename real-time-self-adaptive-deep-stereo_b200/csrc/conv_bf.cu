@@ -1,10 +1,10 @@
-// conv_bf: tcgen05 implicit-GEMM convolution on split 16-bit operands -- the default tensor-core path of the conv stacks.
+// conv_bf: tcgen05 implicit-GEMM convolution on split 16-bit operands -- the tensor-core path of the conv stacks.
 //
 // Replaces the cuDNN calls behind tf.nn.conv2d / tf.nn.atrous_conv2d (reference Nets/sharedLayers.py:58,72) and their
 // input gradients for the estimator / context / pyramid layers of MADNet (Nets/MadNet.py:73-171,173-249) and the
 // DispNet encoder / refinement convs (Nets/DispNet.py:77-140).
 //
-// Why a second tensor-core generation (round-2 findings, DESIGN.md section 4): the 3xTF32 kernels (conv_tc.cu) split
+// Why this tensor-core generation (round-2 findings, DESIGN.md section 4): round 1's 3xTF32 kernels (since removed) split
 // fp32 activations inside the main loop (splitter warps, three-party mbarrier hand-shakes) and every 128-pixel CTA
 // re-streams the whole weight set: 10x L2->SM amplification, tensor pipe < 50 %.  Here
 //   * operands are PRE-SPLIT: every tensor that feeds a convolution also exists as two 16-bit planes (x ~= hi + lo),

@@ -4,8 +4,8 @@
 // (reference Nets/sharedLayers.py:54-92) and the conv gradients tf.gradients derives for them.
 // One "gather GEMM" kernel serves conv forward, conv dgrad and conv_transpose forward (see ConvGemm in
 // common.cuh); a second kernel computes weight gradients as a split-K GEMM over pixels with a
-// deterministic two-pass reduction.  This is the exact-fp32 path: it is used for every layer shape the
-// tcgen05 path (conv_tc.cu) does not cover (stride 2, cin=3, cout=1, transposed) and as its checker.
+// deterministic two-pass reduction.  This is the exact-fp32 path: the generic fallback for every layer shape the
+// split-16-bit tensor-core path (conv_bf.cu, wgrad_bf.cu) does not take, and the op-level reference for it.
 #include "common.cuh"
 #include <algorithm>
 #include <cstdlib>
@@ -245,6 +245,8 @@ __global__ void gemm_splitk_reduce_kernel(ConvGemm p, int M) {
 }
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+size_t conv_gemm_part_floats() { return (size_t)8 << 20; }      // 32 MB; conv_gemm splits K only as far as it fits
 
 int conv_gemm(const ConvGemm& p_in, cudaStream_t st) {
     ConvGemm p = p_in;

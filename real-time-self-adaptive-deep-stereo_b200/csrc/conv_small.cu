@@ -89,7 +89,7 @@ __global__ void __launch_bounds__(CS_NT) conv_small_fwd_kernel(ConvGemm p, int p
         const size_t pix = (size_t)(img * p.y.h + oy) * p.y.w + ox;
         float* yrow = p.y.p + pix * p.y.cs;
 #pragma unroll
-        for (int j = 0; j < CO; ++j) {                       // same epilogue order as conv_gemm_kernel / conv_tc
+        for (int j = 0; j < CO; ++j) {                       // same epilogue order as conv_gemm_kernel
             float t = fmaxf(p.alpha * acc[pi][j], acc[pi][j]);
             if (p.res) t += p.res[pix * p.res_cs + j];
             if (p.accumulate) t += yrow[j];

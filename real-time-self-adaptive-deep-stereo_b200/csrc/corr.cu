@@ -437,7 +437,6 @@ static bool corr_use_tma() {
     if (v < 0) { const char* e = getenv("MS_CORR_NO_TMA"); v = (e && e[0] == '1') ? 0 : 1; }
     return v == 1;
 }
-int corr_init();
 static bool a16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 static int pick_tw(int w, int C, int d, bool warped, size_t row_bufs_full, size_t budget, size_t extra) {

@@ -21,6 +21,8 @@
 #include <algorithm>
 #include <climits>
 #include <cstdlib>
+#include <cstring>
+#include <map>
 
 #include "common.cuh"
 #include "corr_common.cuh"
@@ -253,6 +255,61 @@ __global__ void __launch_bounds__(256) corr_fwd4_kernel(const __grid_constant__ 
 
 static int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
 static bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+static EncodeTiledFn get_encode() {
+    static EncodeTiledFn fn = nullptr;
+    if (!fn) {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult qres;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
+            qres == cudaDriverEntryPointSuccess)
+            fn = reinterpret_cast<EncodeTiledFn>(p);
+    }
+    return fn;
+}
+
+struct MapKey {
+    uintptr_t addr; int rank; int swz; uint64_t d[4]; uint64_t s[3]; uint32_t b[4];
+    bool operator<(const MapKey& o) const { return memcmp(this, &o, sizeof(MapKey)) < 0; }
+};
+
+// fp32 tensor maps for the TMA copies here and in wgrad_tc.cu (declared in tc_ptx.cuh)
+int tc_get_map(const CUtensorMap** out, void* addr, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
+               const cuuint32_t* box, bool swizzle128) {
+    static std::map<MapKey, CUtensorMap> cache;
+    MapKey k;
+    memset(&k, 0, sizeof k);
+    k.addr = reinterpret_cast<uintptr_t>(addr); k.rank = rank; k.swz = swizzle128 ? 1 : 0;
+    for (int i = 0; i < rank; ++i) { k.d[i] = dims[i]; k.b[i] = box[i]; }
+    for (int i = 0; i + 1 < rank; ++i) k.s[i] = strides_bytes[i];
+    auto it = cache.find(k);
+    if (it == cache.end()) {
+        EncodeTiledFn enc = get_encode();
+        MS_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled entry point not available");
+        cuuint32_t es[5] = {1, 1, 1, 1, 1};
+        CUtensorMap m;
+        CUresult r = enc(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank, addr, dims, strides_bytes, box, es,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with code " + std::to_string((int)r)); return -1; }
+        if (cache.size() >= 4096) {
+            // cache full (callers that keep passing fresh pointers): do not evict -- pointers handed out earlier in the same
+            // launch sequence must stay valid -- but serve this descriptor from a small ring of uncached slots
+            static thread_local CUtensorMap spill[16];
+            static thread_local unsigned spill_i = 0;
+            CUtensorMap* slot = &spill[spill_i++ & 15u];
+            *slot = m;
+            *out = slot;
+            return 0;
+        }
+        it = cache.emplace(k, m).first;
+    }
+    *out = &it->second;
+    return 0;
+}
 
 // 3-D view {channels, w, B*h} of an NHWC tensor with channel stride cs; box {32, rows, 1}
 static int feat_map(CUtensorMap* out, const float* ptr, int chans, int cs, int w, int rows_total, int box_rows) {

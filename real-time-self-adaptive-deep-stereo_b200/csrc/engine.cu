@@ -38,27 +38,21 @@ Engine::Engine()
       wg_ws(nullptr), wg_ws_floats(0), rs_tmp(nullptr), rs_tmp_floats(0), loss_ws(nullptr), loss_ws_floats(0),
       scalars(nullptr), gt(nullptr), proxy(nullptr), loss_kind(0), proxy_w_full(0.01f), proxy_w_module(0.1f), profiling(0), prof_capturing(false), prof_event_overhead_ms(0.f) {
     prof_reset();
-    prep_jobs_dev = nullptr; prep_max_total = 0; weights_dirty = true;
+    weights_dirty = true;
     gstream = nullptr; ev_in = nullptr; ev_out = nullptr;
     wstream = nullptr; ev_fork = nullptr; ev_join = nullptr; wstream_dirty = false;
     { const char* e8 = getenv("MS_WGRAD_OVERLAP"); use_overlap = (e8 && e8[0] == '0') ? 0 : 1; }
     { const char* e2 = getenv("MS_GRAPHS"); use_graphs = (e2 && e2[0] == '0') ? 0 : 1; }
-    { const char* e3 = getenv("MS_TC_WGRAD"); use_tc_wgrad = (e3 && e3[0] == '0') ? 0 : 1; }
-    const char* e = getenv("MS_CONV_TC");
-    use_tc = (e && e[0] == '0') ? 0 : 1;
-    { const char* e4 = getenv("MS_CONV_IMPL"); conv_impl = (e4 && (!strcmp(e4, "tf32") || !strcmp(e4, "0"))) ? 0 : 1; }
-    if (!use_tc) conv_impl = 0;
     { const char* e5 = getenv("MS_HEADS"); use_heads = (e5 && e5[0] == '0') ? 0 : 1; }
     { const char* e7 = getenv("MS_STEM"); use_stem = (e7 && e7[0] == '0') ? 0 : 1; }
     { const char* e6 = getenv("MS_BF_WGRAD"); use_bf_wgrad = (e6 && e6[0] == '0') ? 0 : 1; }
     wg_xp.hi = wg_xp.lo = nullptr; wg_xp.cs = 0; wg_xp.fmt = 0; wg_xp.scale = 1.f; wg_xp_halfs = 0;
     act_scale = 0.f;
-    bf_jobs_dev = nullptr; bf_max_total = 0; bf_part = nullptr; bf_tickets = nullptr;
+    bf_jobs_dev = nullptr; bf_max_total = 0; bf_part = nullptr; bf_tickets = nullptr; gemm_part = nullptr;
     dp_rank = 0; dp_world = 1; dp_connected = false; dp_xbuf = nullptr; dp_state = nullptr; dp_cap_floats = 0;
 }
 
 void Engine::add_planes(Bump& A, const TView& v, int fmt) {
-    if (conv_impl != 1) return;
     const bool sizing = A.base == nullptr;         // (sizing pass: pointers are null or null + a slice offset -- never dedupe)
     if (!sizing && planes.count(v.p)) return;
     ActPlanes pl;
@@ -223,7 +217,7 @@ size_t Engine::layout(float* base) {
             max_wg = std::max(max_wg, pixels * L.cout + 64 * (size_t)L.kh * L.kw * L.cin * L.cout + 128 * (size_t)L.cout + 8192);
         max_wt = std::max(max_wt, (size_t)L.kh * L.kw * L.cin * L.cout);
         if (L.cout == 1) max_wg = std::max(max_wg, (size_t)2 * 148 * ((size_t)L.kh * L.kw * L.cin + 1));    // conv_head_wgrad partials
-        if (conv_impl == 1 && !L.transposed && L.cin >= 3 && L.cout >= 16) {
+        if (!L.transposed && L.cin >= 3 && L.cout >= 16) {
             max_wg = std::max(max_wg, std::min<size_t>(wgrad_bf_workspace_floats(L.kh, L.kw, L.cin, L.cout), (size_t)48 << 20));
             wg_xp_halfs = std::max(wg_xp_halfs, pixels * L.stride * L.stride * (size_t)((L.cin + 7) / 8 * 8));
         }
@@ -295,39 +289,12 @@ size_t Engine::layout(float* base) {
     tensors["grad/disp"] = g_disp;
     wT_floats = max_wt; wT = alloc(max_wt);
     wg_ws_floats = max_wg; wg_ws = alloc(max_wg);
-    // persistent tcgen05 weight halves + the batched prep job table
-    tcw[0].assign(layers.size(), TcW{nullptr, nullptr, 0, false});
-    tcw[1].assign(layers.size(), TcW{nullptr, nullptr, 0, false});
-    prep_jobs.clear(); job_begin.assign(n_groups + 1, 0); job_end.assign(n_groups + 1, 0);
-    prep_max_total = 0;
-    for (int gidx = 0; gidx <= n_groups; ++gidx) {
-        job_begin[gidx] = (int)prep_jobs.size();
-        for (size_t li = 0; li < layers.size(); ++li) {
-            const ConvLayer& L = layers[li];
-            const int lg = L.group < 0 ? n_groups : L.group;
-            if (conv_impl == 1) continue;                       // the split-bf16 path has its own weight copies (below)
-            if (lg != gidx || L.transposed || L.stride != 1 || L.cin < 8 || L.cout < 8) continue;
-            for (int dir = 0; dir < 2; ++dir) {
-                const int N = dir == 0 ? L.cout : L.cin, K = dir == 0 ? L.cin : L.cout;
-                if (N > 256 || (long)N * K < 1024) continue;
-                int BN, Kpad; conv_tc_weight_dims(N, K, BN, Kpad);
-                const size_t per = (size_t)L.kh * L.kw * BN * Kpad;
-                TcW t; t.per = per; t.ok = true;
-                t.bh = alloc(per); t.bl = nullptr;
-                tcw[dir][li] = t;
-                TcPrepJob j{base ? Wt + L.w_off : nullptr, t.bh, t.bl, L.kh * L.kw, N, K, BN, Kpad, dir == 0 ? 1 : 0};
-                prep_jobs.push_back(j);
-                prep_max_total = std::max(prep_max_total, per);
-            }
-        }
-        job_end[gidx] = (int)prep_jobs.size();
-    }
     // split 16-bit weight tiles per layer and orientation (forward: fp16, dgrad: bf16) + their batched prep job table
     bfw[0].assign(layers.size(), BfW{nullptr, false});
     bfw[1].assign(layers.size(), BfW{nullptr, false});
     bf_jobs.clear(); bf_job_begin.assign(n_groups + 1, 0); bf_job_end.assign(n_groups + 1, 0);
     bf_max_total = 0;
-    for (int gidx = 0; gidx <= n_groups && conv_impl == 1; ++gidx) {
+    for (int gidx = 0; gidx <= n_groups; ++gidx) {
         bf_job_begin[gidx] = (int)bf_jobs.size();
         for (size_t li = 0; li < layers.size(); ++li) {
             const ConvLayer& L = layers[li];
@@ -374,14 +341,13 @@ size_t Engine::layout(float* base) {
         }
         bf_job_end[gidx] = (int)bf_jobs.size();
     }
-    if (conv_impl == 1 && wg_xp_halfs) {
+    if (wg_xp_halfs) {
         wg_xp.hi = alloc((wg_xp_halfs + 1) / 2); wg_xp.lo = alloc((wg_xp_halfs + 1) / 2); wg_xp.fmt = 0;
     }
     bf_part = alloc(conv_bf_part_floats());
     bf_tickets = reinterpret_cast<unsigned int*>(alloc(conv_bf_ticket_words()));
     bf_jobs_dev = reinterpret_cast<BfPrepJob*>(alloc((bf_jobs.size() + 1) * sizeof(BfPrepJob) / sizeof(float) + 16));
-    tc_part = alloc(conv_tc_part_floats());
-    prep_jobs_dev = reinterpret_cast<TcPrepJob*>(alloc((prep_jobs.size() + 1) * sizeof(TcPrepJob) / sizeof(float) + 16));
+    gemm_part = alloc(conv_gemm_part_floats());
     rs_tmp_floats = (size_t)B * H * Wp; rs_tmp = alloc(rs_tmp_floats);
     loss_ws_floats = loss_workspace_floats(B, H, W); loss_ws = alloc(loss_ws_floats);
     scalars = alloc(64);
@@ -402,7 +368,7 @@ int Engine::conv_fwd(const ConvLayer& L, const TView& x, const TView& y, const f
     p.alpha = L.alpha;
     p.res = res; p.res_cs = res_cs;
     p.mask = nullptr; p.mask_cs = 0; p.mask_alpha = 1.f; p.accumulate = 0;
-    p.part = tc_part; p.part_floats = conv_tc_part_floats();
+    p.part = gemm_part; p.part_floats = conv_gemm_part_floats();
     int oh, ow, pt, pl;
     if (!L.transposed) {
         same_pad(x.h, L.kh, L.stride, L.dil, oh, pt);
@@ -417,14 +383,14 @@ int Engine::conv_fwd(const ConvLayer& L, const TView& x, const TView& y, const f
         p.wmat = wT;
         p.mul = 1; p.off_y = pt; p.off_x = pl; p.step = -1; p.div = L.stride;
         const int li_t = (int)(&L - &layers[0]);
-        const bool bf_t = conv_impl == 1 && bfw[0][li_t].ok && conv_bf_supported(p) && planes_of(x);
+        const bool bf_t = bfw[0][li_t].ok && conv_bf_supported(p) && planes_of(x);
         // canonical W is [tap][cout][cin]; the gather GEMM wants [tap][K=cin][N=cout] (the tensor-core path has its own tiles)
         if (!bf_t && transpose_taps(Wt + L.w_off, wT, L.kh * L.kw, L.cout, L.cin, st)) return -1;
     }
     const int li = (int)(&L - &layers[0]);
     prof_begin(CAT_CONV_FWD, st, li);
     int rc;
-    const ActPlanes* xpl = (conv_impl == 1 && bfw[0][li].ok && conv_bf_supported(p)) ? planes_of(x) : nullptr;
+    const ActPlanes* xpl = (bfw[0][li].ok && conv_bf_supported(p)) ? planes_of(x) : nullptr;
     if (use_heads && conv_head_kind(p) == 1) {
         fresh.erase(y.p);
         rc = conv_head(p, st);
@@ -450,8 +416,7 @@ int Engine::conv_fwd(const ConvLayer& L, const TView& x, const TView& y, const f
         if (ypl) fresh.insert(y.p);
     } else {
         fresh.erase(y.p);
-        if (use_tc && tcw[0][li].ok && conv_tc_profitable(p)) rc = conv_tc(p, tcw[0][li].bh, st, tc_part);
-        else rc = conv_gemm(p, st);
+        rc = conv_gemm(p, st);
     }
     prof_end(st);
     prof_note((double)y.pixels() * L.kh * L.kw * L.cin * L.cout / (L.transposed ? L.stride * L.stride : 1), 0);
@@ -475,7 +440,7 @@ int Engine::conv_bwd(const ConvLayer& L, const TView& x, const TView& dpre, cons
         prof_begin(CAT_CONV_WGRAD, st, (int)(&L - &layers[0]));
         int rc = 0;
         const bool stem_w = use_stem && conv_stem_wgrad_supported(q);
-        const ActPlanes* wxp = (!stem_w && conv_impl == 1 && use_bf_wgrad && wgrad_bf_supported(q)) ? planes_of(x) : nullptr;
+        const ActPlanes* wxp = (!stem_w && use_bf_wgrad && wgrad_bf_supported(q)) ? planes_of(x) : nullptr;
         const ActPlanes* wdp = wxp ? planes_of(dpre) : nullptr;
         // the planes of dpre also feed the dgrad below: they are produced on `st` BEFORE the fork
         if (wxp && wdp) rc = ensure_planes(dpre, st);
@@ -493,7 +458,7 @@ int Engine::conv_bwd(const ConvLayer& L, const TView& x, const TView& dpre, cons
         } else if (!rc && use_heads && conv_head_wgrad_supported(q)) {
             rc = conv_head_wgrad(q, ws);                 // single-channel disparity heads
         } else if (!rc) {
-            rc = (use_tc && use_tc_wgrad && wgrad_tc_supported(q)) ? wgrad_tc(q, ws) : conv_wgrad(q, ws);
+            rc = wgrad_tc_supported(q) ? wgrad_tc(q, ws) : conv_wgrad(q, ws);
         }
         prof_end(st);
         prof_note((double)dpre.pixels() * L.kh * L.kw * L.cin * L.cout, 0);
@@ -506,11 +471,11 @@ int Engine::conv_bwd(const ConvLayer& L, const TView& x, const TView& dpre, cons
         p.alpha = 1.f;
         p.mask = dx_mask ? dx_mask->p : nullptr; p.mask_cs = dx_mask ? dx_mask->cs : 0; p.mask_alpha = mask_alpha;
         p.res = nullptr; p.res_cs = 0; p.accumulate = dx_acc;
-        p.part = tc_part; p.part_floats = conv_tc_part_floats();
+        p.part = gemm_part; p.part_floats = conv_gemm_part_floats();
         const int li = (int)(&L - &layers[0]);
         prof_begin(CAT_CONV_DGRAD, st, li);
         int rc;
-        const ActPlanes* xpl = (conv_impl == 1 && bfw[1][li].ok && conv_bf_supported(p)) ? planes_of(dpre) : nullptr;
+        const ActPlanes* xpl = (bfw[1][li].ok && conv_bf_supported(p)) ? planes_of(dpre) : nullptr;
         if (use_heads && L.cout == 1 && (p.wmat = Wt + L.w_off, conv_head_kind(p) == 2)) {
             fresh.erase(dx->p);
             rc = conv_head(p, st);          // [tap][cin][1] == [tap][1][cin]: the canonical weights serve directly
@@ -520,10 +485,6 @@ int Engine::conv_bwd(const ConvLayer& L, const TView& x, const TView& dpre, cons
             const ActPlanes* ypl = planes_of(*dx);
             if (!rc) rc = conv_bf(p, *xpl, bfw[1][li].tiles, ypl, bf_part, bf_tickets, st);
             if (ypl) fresh.insert(dx->p);
-        } else if (use_tc && tcw[1][li].ok && conv_tc_profitable(p)) {
-            p.wmat = wT;
-            fresh.erase(dx->p);
-            rc = conv_tc(p, tcw[1][li].bh, st, tc_part);
         } else {
             p.wmat = wT;
             fresh.erase(dx->p);
@@ -568,18 +529,11 @@ int Engine::set_input_u8(const unsigned char* left, const unsigned char* right, 
 }
 
 int Engine::prep_layers(int group, cudaStream_t st) {
-    if (!use_tc) return 0;
-    if (!bf_jobs.empty()) {
-        int b, e;
-        if (group < 0) { b = 0; e = (int)bf_jobs.size(); }
-        else { b = bf_job_begin[group]; e = bf_job_end[group]; }
-        if (bf_prep_weights(bf_jobs_dev + b, e - b, bf_max_total, st)) return -1;
-    }
-    if (prep_jobs.empty()) return 0;
+    if (bf_jobs.empty()) return 0;
     int b, e;
-    if (group < 0) { b = 0; e = (int)prep_jobs.size(); }
-    else { b = job_begin[group]; e = job_end[group]; }
-    return tc_prep_weights(prep_jobs_dev + b, e - b, prep_max_total, st);
+    if (group < 0) { b = 0; e = (int)bf_jobs.size(); }
+    else { b = bf_job_begin[group]; e = bf_job_end[group]; }
+    return bf_prep_weights(bf_jobs_dev + b, e - b, bf_max_total, st);
 }
 
 int Engine::forward(int disp_mask, cudaStream_t st) {
@@ -862,7 +816,7 @@ int Engine::update(int group, float lr, float mu, float gscale, cudaStream_t st)
     size_t b = 0, e = n_params;
     if (group >= 0) { MS_REQUIRE(group < n_groups, "update: bad group"); b = group_begin[group]; e = group_end[group]; }
     if (momentum_update(Wt + b, Gr + b, Mo + b, e - b, lr, mu, gscale, st)) return -1;
-    return prep_layers(group, st);      // refresh the tf32 hi/lo copies of exactly the weights that moved
+    return prep_layers(group, st);      // refresh the 16-bit weight tiles of exactly the weights that moved
 }
 
 // forward + losses + backward (+ update) as one sequence; replayed as a CUDA graph after the first call
@@ -894,7 +848,7 @@ int Engine::run(int mode, int group, int disp_mask, int with_update, float lr, f
     MS_REQUIRE(bound, "engine not bound");
     MS_REQUIRE(mode == 0 || mode == 2 || (mode == 1 && group >= 0 && group < n_groups), "run: bad mode/group");
     if (!use_graphs || profiling == 1) return run_eager(mode, group, disp_mask, with_update, lr, mu, gscale, st);
-    if (weights_dirty) {                    // load / restore happened: refresh every tf32 copy outside the graph
+    if (weights_dirty) {                    // load / restore happened: refresh every weight tile outside the graph
         if (prep_layers(-1, st)) return -1;
         weights_dirty = false;
     }
@@ -909,7 +863,7 @@ int Engine::run(int mode, int group, int disp_mask, int with_update, float lr, f
     key.lr = lr; key.mu = mu; key.gs = gscale; key.prof = profiling == 2 ? 1 : 0;
     auto it = graphs.find(key);
     if (it == graphs.end()) {
-        if (conv_tc_init() || conv_bf_init() || wgrad_bf_init() || corr_init() || wgrad_tc_init()) return -1;
+        if (conv_bf_init() || wgrad_bf_init() || corr_init() || wgrad_tc_init()) return -1;
         cudaGraph_t graph = nullptr;
         const long long l0 = launch_count();
         if (profiling == 2) { if (prof_collect()) return -1; }

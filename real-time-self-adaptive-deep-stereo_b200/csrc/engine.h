@@ -67,14 +67,7 @@ struct Engine {
     int n_disp;
     TView g_disp;
     float* wT; size_t wT_floats;     // transposed-weight scratch
-    // tcgen05 weight halves (tf32 hi / lo), persistent per layer and GEMM orientation (0 = forward, 1 = dgrad);
-    // refreshed for a module's layers right after its momentum update, for everything after load/restore.
-    struct TcW { float* bh; float* bl; size_t per; bool ok; };
-    std::vector<TcW> tcw[2];
-    std::vector<TcPrepJob> prep_jobs;            // ordered by group (then ungrouped)
-    std::vector<int> job_begin, job_end;         // per group ranges into prep_jobs; index n_groups = ungrouped
-    TcPrepJob* prep_jobs_dev; size_t prep_max_total;
-    float* tc_part;                              // split-K partial sums of the tcgen05 conv on small maps
+    float* gemm_part;                            // split-K partial sums of the fp32 conv_gemm on small maps
     bool weights_dirty;
     int prep_layers(int group, cudaStream_t st); // -1 = all
     // whole-step CUDA graphs keyed by (mode, group, disp_mask, with_update, lr, mu, gscale)
@@ -84,7 +77,6 @@ struct Engine {
     struct GraphRec { cudaGraphExec_t exec; long long kernels; std::vector<Span>* spans; };
     std::map<GraphKey, GraphRec> graphs;
     int use_graphs;
-    int use_tc_wgrad;                            // MS_TC_WGRAD (default 1)
     cudaStream_t gstream; cudaEvent_t ev_in, ev_out;   // graphs run on a private stream (the legacy default stream cannot be captured)
     // weight gradients on a side stream: wgrad(layer j) only needs dpre_j and the forward activation, so it runs concurrently
     // with the dgrad chain (fork / join through events; inside the captured step this becomes a parallel graph branch)
@@ -95,12 +87,10 @@ struct Engine {
     int backward_impl(int mode, int group, cudaStream_t st);
     int run(int mode, int group, int disp_mask, int with_update, float lr, float mu, float gscale, cudaStream_t st);
     int run_eager(int mode, int group, int disp_mask, int with_update, float lr, float mu, float gscale, cudaStream_t st);
-    int use_tc;                      // route eligible convs through conv_tc (env MS_CONV_TC, default 1)
-    // ---- split-bf16 tcgen05 path (conv_bf.cu), the default implementation of every eligible conv / dgrad
+    // ---- split-bf16 tcgen05 path (conv_bf.cu), the implementation of every eligible conv / dgrad
     int use_stem;                                  // direct CUDA-core kernels for DispNet conv1 (MS_STEM=0: tensor-core path)
     int use_bf_wgrad;                              // split-bf16 weight gradients (MS_BF_WGRAD=0: the 3xTF32 / fp32 kernels)
     int use_heads;                                 // direct kernels for the 3x3 -> 1 heads (MS_HEADS=0: generic path)
-    int conv_impl;                                 // 1 = split-bf16 (default), 0 = the 3xTF32 kernels (MS_CONV_IMPL=tf32)
     std::map<const float*, ActPlanes> planes;      // bf16 hi/lo planes of tensors that feed convolutions (key: base pointer)
     std::set<const float*> fresh;                  // planes already written by a conv_bf epilogue in the current pass
     struct BfW { void* tiles; bool ok; };

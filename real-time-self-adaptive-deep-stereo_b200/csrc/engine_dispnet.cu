@@ -56,11 +56,11 @@ void Engine::layout_dispnet(Bump& A, size_t& max_wg, size_t& max_wt) {
         max_wt = std::max(max_wt, (size_t)L.kh * L.kw * L.cin * L.cout);
         if (L.cout == 1) max_wg = std::max(max_wg, (size_t)2 * 148 * ((size_t)L.kh * L.kw * L.cin + 1));    // conv_head_wgrad partials
         if (L.kh == 7 && L.cin == 3 && L.cout == 64) max_wg = std::max(max_wg, (size_t)2 * 148 * (147 * 64 + 64));   // conv_stem_wgrad partials
-        if (conv_impl == 1 && !L.transposed && L.cin >= 3 && L.cout >= 16) {
+        if (!L.transposed && L.cin >= 3 && L.cout >= 16) {
             max_wg = std::max(max_wg, std::min<size_t>(wgrad_bf_workspace_floats(L.kh, L.kw, L.cin, L.cout), (size_t)48 << 20));
             wg_xp_halfs = std::max(wg_xp_halfs, pixels * L.stride * L.stride * (size_t)((L.cin + 7) / 8 * 8));
         }
-        if (conv_impl == 1 && L.transposed && L.cin >= 16 && L.cout >= 8) {
+        if (L.transposed && L.cin >= 16 && L.cout >= 8) {
             // conv2d_transpose: its weight gradient is the wgrad of the stride-2 conv big map (cout) -> small map (cin);
             // `pixels` counts the big map, the bf16 scratch copy is of the small one (the layer's forward input)
             max_wg = std::max(max_wg, std::min<size_t>(wgrad_bf_workspace_floats(L.kh, L.kw, L.cout, L.cin), (size_t)48 << 20));
@@ -126,7 +126,7 @@ int Engine::forward_dispnet(int disp_mask, cudaStream_t st) {
         cf.left = c2a.p; cf.lcs = c2a.cs; cf.right = c2b.p; cf.rcs = c2b.cs; cf.u = nullptr; cf.ucs = 0;
         cf.out = d_cat3.p; cf.ocs = d_cat3.cs; cf.out2 = nullptr; cf.o2cs = 0;
         cf.B = B; cf.h = d_c2.h; cf.w = d_c2.w; cf.C = 128; cf.max_disp = DN_MAXD; cf.stride = 1; cf.copy_left = 0; cf.u_chan = 0;
-        cf.plane_scale = conv_impl == 1 ? act_scale : 0.f;   // same fp16 hi/lo arithmetic as the forward convs
+        cf.plane_scale = act_scale;   // same fp16 hi/lo arithmetic as the forward convs
         prof_begin(CAT_CORR_FWD, st);
         int rc = corr_fwd(cf, st);
         prof_end(st);
@@ -174,7 +174,7 @@ int Engine::deconv_bwd(const ConvLayer& L, const TView& x, const TView& dpre, co
     total = std::max((x.w - 1) * L.stride + L.kw - dpre.w, 0);
     const int pl = total / 2;
     const int li = (int)(&L - &layers[0]);
-    const ActPlanes* dpl = conv_impl == 1 ? planes_of(dpre) : nullptr;       // bf16 planes of the big map's gradient
+    const ActPlanes* dpl = planes_of(dpre);       // bf16 planes of the big map's gradient
     if (dpl) { fresh.erase(dpre.p); if (ensure_planes(dpre, st)) return -1; }
     {
         ConvWgrad q{};
@@ -204,7 +204,7 @@ int Engine::deconv_bwd(const ConvLayer& L, const TView& x, const TView& dpre, co
         p.x = dpre; p.wmat = Wt + L.w_off; p.bias = nullptr; p.y = *dx; p.kh = L.kh; p.kw = L.kw;
         p.mul = L.stride; p.off_y = -pt; p.off_x = -pl; p.step = 1; p.div = 1;
         p.alpha = 1.f; p.mask = nullptr; p.mask_alpha = 1.f; p.res = nullptr; p.accumulate = dx_acc;
-        p.part = tc_part; p.part_floats = conv_tc_part_floats();
+        p.part = gemm_part; p.part_floats = conv_gemm_part_floats();
         prof_begin(CAT_CONV_DGRAD, st, li);
         int rc;
         if (dpl && bfw[1][li].ok && conv_bf_supported(p)) {

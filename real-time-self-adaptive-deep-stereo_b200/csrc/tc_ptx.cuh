@@ -1,4 +1,5 @@
-// tcgen05 / TMA / mbarrier PTX wrappers shared by the tensor-core kernels (conv_tc.cu, wgrad_tc.cu).
+// tcgen05 / TMA / mbarrier PTX wrappers shared by the tensor-core kernels (conv_bf.cu, wgrad_bf.cu, wgrad_tc.cu) and the
+// TMA-staged correlation (corr_tma.cu).
 #pragma once
 #include <cuda.h>
 
@@ -61,26 +62,8 @@ __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence:
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-__device__ __forceinline__ void tc_mma_tf32(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-        : "memory");
-}
 __device__ __forceinline__ void tc_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s_addr(bar)) : "memory");
-}
-__device__ __forceinline__ void tc_ld16(uint32_t taddr, float (&v)[16]) {
-    uint32_t r[16];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
 }
 
 __device__ __forceinline__ void tc_mma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
@@ -120,14 +103,9 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_byte_addr) {
 // instruction sequence cvt.rna.tf32.f32 expands to -- ncu showed the splitter loop to be instruction-latency bound
 // (349 instructions per warp per K step, 128 of them from the 32 cvt.rna).
 __device__ __forceinline__ float tf32_hi(float x) { return __uint_as_float(__float_as_uint(x) & 0xffffe000u); }
-__device__ __forceinline__ float tf32_rna(float x) {
-    uint32_t r;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-    return __uint_as_float(r);
-}
 
 
-// cached cuTensorMapEncodeTiled (fp32, zero OOB fill); swizzle128=false => SWIZZLE_NONE.  (conv_tc.cu)
+// cached cuTensorMapEncodeTiled (fp32, zero OOB fill); swizzle128=false => SWIZZLE_NONE.  (corr_tma.cu)
 int tc_get_map(const CUtensorMap** out, void* addr, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
                const cuuint32_t* box, bool swizzle128);
 

@@ -13,7 +13,7 @@
 //              forms the tf32 hi/lo halves and writes them to TENSOR MEMORY (tcgen05.st) -> TS-mode MMAs.
 //   B (dY^T) : dY is first transposed to NCHW (one small kernel) so that a TMA box {32,1,N,1} lands as the K-major
 //              SWIZZLE_128B tile [N rows][32 pixels]; hi/lo split in shared memory.
-//   3xTF32 with separated accumulators exactly as in conv_tc.cu (cross terms | rotating hi*hi partial sums).
+//   3xTF32 with separated accumulators (cross terms | rotating hi*hi partial sums).
 // Partial sums [split][tap][ci][co] go to the workspace; the existing fixed-order wgrad_reduce finishes (deterministic).
 #include <algorithm>
 #include <cstdlib>

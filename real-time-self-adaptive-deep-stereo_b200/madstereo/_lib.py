@@ -29,9 +29,6 @@ _SIGS = {
     'ms_corr_bwd': (I, [P, I, P, I, P, I, P, I, P, I, P, I, P, I, I, I, I, I, I, I, I, P]),
     'ms_conv2d_fwd': (I, [P, I, I, I, I, I, P, P, P, I, I, I, I, I, I, F, P]),
     'ms_conv2d_dgrad': (I, [P, I, I, I, I, I, P, P, I, I, I, I, I, I, I, I, P, P]),
-    'ms_conv2d_fwd_tc': (I, [P, I, I, I, I, I, P, P, P, I, I, I, I, I, F, P, Z, P]),
-    'ms_conv2d_dgrad_tc': (I, [P, I, I, I, I, I, P, P, I, I, I, I, I, P, Z, P]),
-    'ms_conv2d_tc_scratch': (Z, [I, I, I, I]),
     'ms_conv2d_fwd_bf': (I, [P, I, I, I, I, I, P, P, P, I, I, I, I, I, I, F, F, P, Z, P]),
     'ms_conv2d_dgrad_bf': (I, [P, I, I, I, I, I, P, P, I, I, I, I, I, I, I, I, P, Z, P]),
     'ms_conv2d_bf_scratch': (Z, [I, I, I, I, I, I, I]),
@@ -94,7 +91,6 @@ _SIGS = {
     'ms_engine_profile_layers': (I, [P, P, P]),
     'ms_engine_profile_event_overhead_ms': (F, [P]),
     'ms_launch_count': (ctypes.c_longlong, []),
-    'ms_debug_tc_prof': (I, [POINTER(ctypes.c_ulonglong), I]),
     'ms_debug_bf_prof': (I, [P, I]),
     'ms_engine_num_tensors': (I, [P]),
     'ms_engine_tensor_name': (I, [P, I, c_char_p, I]),

@@ -103,29 +103,6 @@ def conv2d(x, w, b, stride=1, dilation=1, alpha=1.0):
     return y
 
 
-def conv2d_tc(x, w, b, dilation=1, alpha=1.0):
-    """tcgen05 / 3xTF32 forward of a stride-1 conv (same semantics as conv2d)."""
-    n, h, wd, cin = x.shape
-    kh, kw, _, cout = w.shape
-    y = torch.empty(n, h, wd, cout, device=x.device, dtype=torch.float32)
-    ns = lib().ms_conv2d_tc_scratch(kh, kw, cin, cout)
-    scratch = torch.empty(ns, device=x.device, dtype=torch.float32)
-    check(lib().ms_conv2d_fwd_tc(_p(x), n, h, wd, cin, cin, _p(w), _p(b), _p(y), cout, cout, kh, kw, dilation,
-                                 float(alpha), _p(scratch), ns, _s()), 'ms_conv2d_fwd_tc')
-    return y
-
-
-def conv2d_dgrad_tc(dy, w, dilation=1):
-    n, h, wd, cout = dy.shape
-    kh, kw, cin, _ = w.shape
-    dx = torch.empty(n, h, wd, cin, device=dy.device, dtype=torch.float32)
-    ns = lib().ms_conv2d_tc_scratch(kh, kw, cin, cout)
-    scratch = torch.empty(ns, device=dy.device, dtype=torch.float32)
-    check(lib().ms_conv2d_dgrad_tc(_p(dy), n, h, wd, cout, cout, _p(w), _p(dx), cin, cin, kh, kw, dilation,
-                                   _p(scratch), ns, _s()), 'ms_conv2d_dgrad_tc')
-    return dx
-
-
 def conv2d_bf(x, w, b, stride=1, dilation=1, alpha=1.0, act_scale=0.0625):
     """split-bf16 tcgen05 forward conv (csrc/conv_bf.cu; same semantics as conv2d, stride 1 or 2)."""
     n, h, wd, cin = x.shape

@@ -46,25 +46,21 @@ def main():
     import Nets
     from madstereo.adaptation import OnlineAdaptation
     cfg = json.load(open(os.path.join(PKG, 'block_config', 'MadNet_full.json')))
-    for name, env in (('gpu_fp16x3_fwd_bf16x3_bwd (shipped)', {}), ('gpu_3xTF32 (MS_CONV_IMPL=tf32)', {'MS_CONV_IMPL': 'tf32'})):
-        for k in ('MS_CONV_IMPL',):
-            os.environ.pop(k, None)
-        os.environ.update(env)
-        l0 = torch.from_numpy(frames[0][0]).cuda(); r0 = torch.from_numpy(frames[0][1]).cuda()
-        sys.stdout, real = sys.stderr, sys.stdout
-        net = Nets.get_stereo_net('MADNet', dict(left_img=l0, right_img=r0, split_layers=[None], sequence=True, train_portion='BEGIN',
-                                                 bulkhead=True, warping=True, context_net=True, radius_d=2, stride=1, is_training=False))
-        ad = OnlineAdaptation(net, mode='MAD', train_config=cfg, lr=1e-4, sample_mode='SEQUENTIAL', num_blocks=1, ssim_th=10.0)
-        sys.stdout = real
-        ad.load_weights(params)
-        losses = []
-        for t in range(STEPS):
-            l, r = frames[t % 4]
-            o = ad.step(torch.from_numpy(l).cuda(), torch.from_numpy(r).cuda(), want_disp_mask=0b100000)
-            losses.append(o['loss'])
-        runs[name] = {'w': {k: v.astype(np.float64) for k, v in net.engine.export_params().items()}, 'loss': losses,
-                      'disp': net.get_disparities()[-1].numpy()}
-        del ad, net
+    name = 'gpu_fp16x3_fwd_bf16x3_bwd (shipped)'
+    l0 = torch.from_numpy(frames[0][0]).cuda(); r0 = torch.from_numpy(frames[0][1]).cuda()
+    sys.stdout, real = sys.stderr, sys.stdout
+    net = Nets.get_stereo_net('MADNet', dict(left_img=l0, right_img=r0, split_layers=[None], sequence=True, train_portion='BEGIN',
+                                             bulkhead=True, warping=True, context_net=True, radius_d=2, stride=1, is_training=False))
+    ad = OnlineAdaptation(net, mode='MAD', train_config=cfg, lr=1e-4, sample_mode='SEQUENTIAL', num_blocks=1, ssim_th=10.0)
+    sys.stdout = real
+    ad.load_weights(params)
+    losses = []
+    for t in range(STEPS):
+        l, r = frames[t % 4]
+        o = ad.step(torch.from_numpy(l).cuda(), torch.from_numpy(r).cuda(), want_disp_mask=0b100000)
+        losses.append(o['loss'])
+    runs[name] = {'w': {k: v.astype(np.float64) for k, v in net.engine.export_params().items()}, 'loss': losses,
+                  'disp': net.get_disparities()[-1].numpy()}
     ref = runs['oracle_fp64']
     table = {}
     for name, r in runs.items():
